@@ -53,6 +53,7 @@ REC = 256
 MODEXP_BATCH, K, EL, MODEXP_SEED = 65536, 64, 64, 0xB2000002
 W_MODEXP = 1.2 * 2048 * (2 * K * K + K)
 Q = 0xFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFEBAAEDCE6AF48A03BBFD25E8CD0364141
+DUMP_BYTES, DUMP_SEED = 60 << 20, 0xB200D      # --dump-outputs: budget (under 64 MB with the .npy headers) and row-sample seed
 
 
 def config_dict(world: int) -> dict:
@@ -149,6 +150,21 @@ def load_keysets():
     ks = fixtures.load_all_keysets()
     assert len(ks) == 8, "tests/golden/keys_t1n3.json must hold the 8 key sets of config 5"
     return ks
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write every array as out_dir/<name>.npy: bytes as float32 and 32-bit limbs as float64, both exact.  When the set exceeds
+    DUMP_BYTES, each array keeps its share of the budget as a fixed, seeded sample of rows whose indices go to <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.astype(np.float32 if v.dtype.itemsize == 1 else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, int(DUMP_BYTES * a.nbytes / total) // (a.nbytes // a.shape[0] + 8))
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(a.shape[0], keep, replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_batch(keysets, n_sessions: int, rank: int):
@@ -278,7 +294,12 @@ def main():
     ap.add_argument("--sessions", type=int, default=SESSIONS_PER_GPU, help=argparse.SUPPRESS)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-modexp", action="store_true", help="skip the secondary modexp block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy: rank 0's per-unit status, R, sigma, t_vec, digest "
+                         "and every rank's gathered 256-byte records")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -364,6 +385,10 @@ def main():
     macs_per_step = eng.work() / args.steps
     clocks = sampler.stop() if rank == 0 else None
     dev_records = d_all[rank].cpu().numpy().copy()
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = {"status": d_status, "R": d_R, "sigma": d_sigma, "t_vec": d_tvec, "digest": d_digest, "records": d_all.reshape(world * U, REC)}
+        outputs = {k: v.cpu().numpy().view(np.uint32 if v.dtype == torch.int32 else np.uint8) for k, v in outputs.items()}
 
     # ---- per-launch durations of the job kernels (CUDA events around every launch, one extra step, single stream)
     prof = eng.profile_step(step_device)
@@ -404,7 +429,7 @@ def main():
     modexp = None
     if not args.no_modexp:
         try:
-            modexp, _, _ = bench_modexp(eng, pkg, torch, rank, max(1, min(args.steps, 3)), threads, check=(rank == 0))
+            modexp, _, _ = bench_modexp(eng, pkg, torch, rank, args.steps, threads, check=(rank == 0))
         except Exception as exc:
             modexp = {"error": f"{type(exc).__name__}: {exc}"}
 
@@ -491,6 +516,8 @@ def main():
         "modexp": modexp,
     }
     print(json.dumps(line), flush=True)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if comm is not None:
         eng.nccl_comm_destroy(comm)
     if world > 1:
