@@ -9,6 +9,7 @@
 #include "gg20_rounds.cuh"
 #include "modinv.cuh"
 
+#include <algorithm>
 #include <cstdlib>
 #include <string>
 #include <thread>
@@ -25,6 +26,8 @@ struct Builder {
     int U;
     ExpLaunch L32, L64, L128, LPQ;      // 1024-bit, 2048-bit, N-adic mod N^2, p-adic mod p^2 / q^2
     InvLaunch I64, I128, I128H;        // I128H: modulo N^2 via the N-wide inversion + Hensel step
+    const uint32_t* order[2];          // units ordered by own / peer key row (keyexp.h), order_len[r] slots each
+    int order_len[2];
 
     Operand fld(int f, int limbs = 0) const {
         return Operand{A.base + (size_t)A.off[f] * U, nullptr, A.size[f], 0, (uint32_t)(limbs ? limbs : A.size[f])};
@@ -56,13 +59,20 @@ struct Builder {
             dst = &LPQ; gpw = 32 / tecdsa_nadic32_tpi(); wide0 = 0;      // operand width is handled by the lift (any width up to 4K)
             mod = key(is_p ? KT_P : KT_Q, mod.idx); nadic = Operand{is_p ? ks->nadic_p : ks->nadic_q, mod.idx, NADIC_ROW * 32, 1, NADIC_ROW * 32};
         }
+        // base 0 raised to an exponent of the own or the peer key row: the class runs over the units ordered by that row, so
+        // that its warps are key-uniform and can walk the row's sliding-window schedule
+        int kx = -1;
+        if (nb > 0 && (e0.idx == A.row_own || e0.idx == A.row_peer))
+            for (int t : {KT_N, KT_P, KT_Q, KT_PM1, KT_QM1, KT_QMODPM1, KT_PMODQM1})
+                if (e0.ptr == A.key[t]) kx = e0.idx == A.row_peer;
         ExpClass& k = dst->cls[dst->n_classes++];
         k.mod = mod; k.base[0] = b0; k.base[1] = b1; k.exp[0] = e0; k.exp[1] = e1; k.exp_limbs[0] = el0; k.exp_limbs[1] = el1;
         k.mul[0] = m0; k.mul[1] = m1; k.mul[2] = m2; k.nbases = nb; k.nmul = nm; k.wide0 = wide0;
         k.fb = nullptr; k.fb_row = Operand{nullptr, nullptr, 0, 0, 0}; k.fb_sel[0] = k.fb_sel[1] = 0;
         k.nadic = nadic;
-        k.out = out(out_field); k.out_stride = A.size[out_field]; k.count = U; k.item_begin = dst->total_items;
-        dst->total_items += (U + gpw - 1) / gpw;
+        k.order = kx >= 0 ? order[kx] : nullptr; k.keyexp = kx >= 0;
+        k.out = out(out_field); k.out_stride = A.size[out_field]; k.count = kx >= 0 ? order_len[kx] : U; k.item_begin = dst->total_items;
+        dst->total_items += (k.count + gpw - 1) / gpw;
     }
     // out = [m0 *] h2^e_h2 * h1^e_h1 mod N_tilde(rows) through the per-key fixed-base tables
     void fb_class(ExpLaunch& l, int gpw, const uint32_t* rows, Operand e_h2, int el_h2, Operand e_h1, int el_h1, int nm, Operand m0, int out_field) {
@@ -255,8 +265,12 @@ static int offline_impl(tecdsa_ctx* c, const tecdsa_keyset* ks, const uint32_t* 
     CK(cudaSetDevice(c->device));
     const int U = (int)n_sessions * 2;
 
-    // ---- host-side unit tables (who am I, who is my peer, which key rows)
-    std::vector<uint32_t> idx((size_t)7 * U);
+    // ---- host-side unit tables (who am I, who is my peer, which key rows), then the units ordered by own and by peer key row,
+    // each row's run padded to whole warps of every job kernel (groups per warp are powers of two: the largest covers all)
+    const uint32_t nrows = (uint32_t)ks->n_keysets * 3;
+    const size_t pad = (size_t)std::max({32 / tecdsa_nadic_tpi(), 32 / tecdsa_nadic32_tpi(), GPW32});
+    const size_t order_cap = (size_t)U + std::min((size_t)nrows, (size_t)U) * (pad - 1);
+    std::vector<uint32_t> idx((size_t)7 * U + 2 * order_cap);
     uint32_t *row_own = idx.data(), *row_peer = row_own + U, *row_st = row_peer + U, *peer = row_st + 3 * (size_t)U, *kset = peer + U;
     for (size_t s = 0; s < n_sessions; s++) {
         uint32_t k = h_sess[3 * s], a = h_sess[3 * s + 1], b = h_sess[3 * s + 2];
@@ -267,6 +281,12 @@ static int offline_impl(tecdsa_ctx* c, const tecdsa_keyset* ks, const uint32_t* 
             for (int x = 0; x < 3; x++) row_st[(size_t)x * U + u] = k * 3 + x;
             peer[u] = (uint32_t)(u ^ 1); kset[u] = k;
         }
+    }
+    size_t order_len[2];
+    {
+        std::vector<uint32_t> scratch(nrows);
+        for (int r = 0; r < 2; r++)
+            order_len[r] = keyexp_order(r ? row_peer : row_own, (size_t)U, nrows, pad, scratch.data(), kset + U + (size_t)r * order_cap);
     }
     // ---- arena
     Builder B;
@@ -282,7 +302,8 @@ static int offline_impl(tecdsa_ctx* c, const tecdsa_keyset* ks, const uint32_t* 
     A.U = U;
     uint32_t* d_idx = reinterpret_cast<uint32_t*>(c->arena + ((arena_bytes + 255) & ~size_t(255)));
     A.row_own = d_idx; A.row_peer = d_idx + U; A.row_st = d_idx + 2 * (size_t)U; A.peer = d_idx + 5 * (size_t)U; A.keyset = d_idx + 6 * (size_t)U;
-    A.status = reinterpret_cast<uint8_t*>(d_idx + 7 * (size_t)U);
+    for (int r = 0; r < 2; r++) { B.order[r] = d_idx + 7 * (size_t)U + (size_t)r * order_cap; B.order_len[r] = (int)order_len[r]; }
+    A.status = reinterpret_cast<uint8_t*>(d_idx + idx.size());
     for (int t = 0; t < KT_COUNT; t++) A.key[t] = ks->tab[t];
     A.ypk = ks->ypk;
     CK(cudaMemcpyAsync(d_idx, idx.data(), idx_bytes, cudaMemcpyHostToDevice, c->stream));
@@ -337,18 +358,18 @@ static int offline_impl(tecdsa_ctx* c, const tecdsa_keyset* ks, const uint32_t* 
     // peer's PDL proof in round 5 (declared shortcut, identical value)
     B.inv_class(I128, GPWI128, B.key(KT_NN, rp), B.peer(F_CK), F_CINVP, 3);
     RUN(run_inv(c, I128, 128)); RUN(run_inv(c, B.I128H, -128));
-    for (int x = 0; x < 3; x++) {
+    for (int x = 0; x < 3; x++)
         B.exp_class(L64, GPW64, B.key(KT_NT, st_rows(x)), 1, B.peer(F_Z0 + x), B.peer(F_E0 + x), 8, NONE, NONE, 0, 0, NONE, NONE, F_ZE0 + x);   // z^e (:122)
-        B.exp_class(L128, GPW128, B.key(KT_NN, rp), 1, B.fld(F_CINVP), B.peer(F_E0 + x), 8, NONE, NONE, 0, 0, NONE, NONE, F_CEI0 + x);           // (c^-1)^e (:135)
-    }
-    RUN(run_exp(c, L128, 128)); RUN(run_exp(c, B.LPQ, -32)); RUN(run_exp(c, L64, 64));
+    RUN(run_exp(c, L64, 64));
     for (int x = 0; x < 3; x++) B.inv_class(I64, GPW64, B.key(KT_NT, st_rows(x)), B.fld(F_ZE0 + x), F_ZEI0 + x, x);
     RUN(run_inv(c, I64, 64));
     for (int x = 0; x < 3; x++) {
         // w' = h1^s1 * h2^s2 * (z^e)^-1 mod N_tilde                     (range_proofs.rs:129-132)
         B.fb_class(L64, GPW64, st_rows(x), B.peer(F_S20 + x), 92, B.peer(F_S10 + x), 28, 1, B.fld(F_ZEI0 + x), F_WV0 + x);
         // u' = (s1 N + 1) * s^N * (c^e)^-1 mod N^2                      (range_proofs.rs:134-141)
-        B.exp_class(L128, GPW128, B.key(KT_NN, rp), 1, B.peer(F_S0 + x, 64), B.key(KT_N, rp), 64, NONE, NONE, 0, 2, B.fld(F_GS10 + x), B.fld(F_CEI0 + x), F_UV0 + x);
+        // (c^-1)^e (:135) is the second base of the same product: its 256-bit exponent shares the squarings of s^N
+        B.exp_class(L128, GPW128, B.key(KT_NN, rp), 2, B.peer(F_S0 + x, 64), B.key(KT_N, rp), 64, B.fld(F_CINVP), B.peer(F_E0 + x), 8, 1,
+                    B.fld(F_GS10 + x), NONE, F_UV0 + x);
     }
     // c_b = c_a^b * Enc(beta'; r') mod N^2 for b = gamma_i and b = w_i  (mta/mod.rs:133-145)
     B.exp_class(L128, GPW128, B.key(KT_NN, rp), 2, B.rnd(RND_R_G, 64), B.key(KT_N, rp), 64, B.peer(F_CK), B.rnd(RND_GAMMA, 8), 8, 1, B.fld(F_LBG), NONE, F_CBG);
@@ -390,16 +411,14 @@ static int offline_impl(tecdsa_ctx* c, const tecdsa_keyset* ks, const uint32_t* 
     B.inv_class(I128, GPWI128, B.key(KT_NN, ro), B.fld(F_CK), F_CINVO, 8);          // own ciphertext (proof j = 0); the peer's inverse is CINVP
     RUN(run_inv(c, I128, 128)); RUN(run_inv(c, B.I128H, -128));
     for (int j = 0; j < 2; j++) {
-        const uint32_t* prover = j ? rp : ro;            // key row of the prover
         const uint32_t* stmt = j ? ro : rp;              // whose (N_tilde, h1, h2) the proof was made against
         Operand z = j ? B.peer(F_PZ) : B.fld(F_PZ);
         B.exp_class(L64, GPW64, B.key(KT_NT, stmt), 1, z, B.fld(F_VE0 + j), 8, NONE, NONE, 0, 0, NONE, NONE, F_VZE0 + j);       // z^e; (z^-1)^e == (z^e)^-1 (:166-172)
-        B.exp_class(L128, GPW128, B.key(KT_NN, prover), 1, B.fld(j ? F_CINVP : F_CINVO), B.fld(F_VE0 + j), 8, NONE, NONE, 0, 0, NONE, NONE, F_VCEI0 + j);  // (c^-1)^e (:151-157)
     }
     B.crt_stage1(L32, GPW32, ro, 5, B.fld(F_PS2, 64));       // own proof's s2^N mod N^2_own through the CRT stages
     RUN(run_exp(c, L32, 32));
     B.crt_stage2(L64, GPW64, ro, 5);
-    RUN(run_exp(c, L128, 128)); RUN(run_exp(c, B.LPQ, -32)); RUN(run_exp(c, L64, 64));
+    RUN(run_exp(c, B.LPQ, -32)); RUN(run_exp(c, L64, 64));
     RUN(glue_crt(c, A, 5, 1));
     for (int j = 0; j < 2; j++) B.inv_class(I64, GPW64, B.key(KT_NT, j ? ro : rp), B.fld(F_VZE0 + j), F_VZEI0 + j, 6 + j);
     RUN(run_inv(c, I64, 64));
@@ -409,9 +428,10 @@ static int offline_impl(tecdsa_ctx* c, const tecdsa_keyset* ks, const uint32_t* 
         Operand s1 = j ? B.peer(F_PS1) : B.fld(F_PS1), s2 = j ? B.peer(F_PS2, 64) : B.fld(F_PS2, 64), s3 = j ? B.peer(F_PS3) : B.fld(F_PS3);
         // u3' = h1^s1 * h2^s3 * z^-e mod N_tilde                         (:158-172)
         B.fb_class(L64, GPW64, stmt, s3, 92, s1, 28, 1, B.fld(F_VZEI0 + j), F_VU30 + j);
-        // u2' = (N+1)^s1 * s2^N * c^-e mod N^2                           (:144-157)
-        if (j == 0) B.exp_class(L128, GPW128, B.key(KT_NN, prover), 0, NONE, NONE, 0, NONE, NONE, 0, 3, B.fld(F_VLIN0), B.fld(F_VCEI0), F_VU20, 0, B.fld(F_XC5));
-        else B.exp_class(L128, GPW128, B.key(KT_NN, prover), 1, s2, B.key(KT_N, prover), 64, NONE, NONE, 0, 2, B.fld(F_VLIN0 + j), B.fld(F_VCEI0 + j), F_VU20 + j);
+        // u2' = (N+1)^s1 * s2^N * c^-e mod N^2                           (:144-157); (c^-1)^e (:151-157) is a base of the same
+        // product.  The own proof's s2^N came through the CRT stages (XC5); the peer's shares its squarings with (c^-1)^e.
+        if (j == 0) B.exp_class(L128, GPW128, B.key(KT_NN, prover), 1, B.fld(F_CINVO), B.fld(F_VE0), 8, NONE, NONE, 0, 2, B.fld(F_VLIN0), B.fld(F_XC5), F_VU20);
+        else B.exp_class(L128, GPW128, B.key(KT_NN, prover), 2, s2, B.key(KT_N, prover), 64, B.fld(F_CINVP), B.fld(F_VE1), 8, 1, B.fld(F_VLIN1), NONE, F_VU21);
     }
     RUN(run_exp(c, L128, 128)); RUN(run_exp(c, B.LPQ, -32)); RUN(run_exp(c, L64, 64));
     RUN(glue(c, gg20_r5_check, A, 2));

@@ -32,7 +32,7 @@ enum : int {
     X(S0, 64) X(S1, 64) X(S2, 64)                                                                 \
     /* round 1: verification of the peer's three range proofs + the two MessageB */               \
     X(ZE0, 64) X(ZE1, 64) X(ZE2, 64) X(CINVP, 128) X(CINVO, 128)   /* c_peer^-1, c_own^-1 mod N^2 */  \
-    X(ZEI0, 64) X(ZEI1, 64) X(ZEI2, 64) X(CEI0, 128) X(CEI1, 128) X(CEI2, 128)                    \
+    X(ZEI0, 64) X(ZEI1, 64) X(ZEI2, 64)                                                           \
     X(GS10, 128) X(GS11, 128) X(GS12, 128)                                                        \
     X(WV0, 64) X(WV1, 64) X(WV2, 64) X(UV0, 128) X(UV1, 128) X(UV2, 128)                          \
     X(LBG, 128) X(LBW, 128) X(CBG, 128) X(CBW, 128)                                               \
@@ -48,7 +48,7 @@ enum : int {
     X(PE, 8) X(PS1, 28) X(PS2, 64) X(PS3, 92)                                                     \
     /* round 5: j = 0 own proof, j = 1 the peer's proof */                                        \
     X(VE0, 8) X(VE1, 8) X(VLIN0, 128) X(VLIN1, 128) X(VZE0, 64) X(VZE1, 64) \
-    X(VZEI0, 64) X(VZEI1, 64) X(VCEI0, 128) X(VCEI1, 128) X(VU20, 128) X(VU21, 128) X(VU30, 64) X(VU31, 64) \
+    X(VZEI0, 64) X(VZEI1, 64) X(VU20, 128) X(VU21, 128) X(VU30, 64) X(VU31, 64)                    \
     X(SI, 16) X(HEG, 48)                            /* T 16 | A3 16 | z1 8 | z2 8 */             \
     X(DIGEST, 8)                                                                                  \
     X(FLAGS, 8)                                     /* one ok byte per check, see gg20_glue.cuh */          \

@@ -12,6 +12,7 @@
 // (src/utilities/zk_pdl_with_slack/mod.rs:182-199).  The two powers share their squarings
 // (Straus interleaving); multipliers m1, m2 are plain residues.
 #pragma once
+#include "keyexp.h"
 #include "modexp.cuh"
 
 namespace tecdsa {
@@ -62,6 +63,10 @@ struct ExpClass {
     // N-adic mode (nadic.cuh, nadic_jobs_kernel only): the job is modulo N^2, `mod` names N and this the key's
     // constants row (digits of R, R^2, R^3 mod N^2)
     Operand nadic;
+    // key-row order (keyexp.h): slot g runs unit order[g] & ~ORDER_PAD and stores only without the ORDER_PAD flag; count is
+    // then the number of slots.  nullptr: slot g runs unit g.
+    const uint32_t* order;
+    int keyexp;             // exp[0] is a key-row exponent and the class is ordered: base 0 runs sliding windows over odd powers
     int count;              // instances
     int item_begin;         // first warp-item of this class in the launch (prefix sum)
 };
@@ -83,6 +88,42 @@ struct ExpLaunch {
     int n_classes;
     int total_items;
 };
+
+// The unit slot g of class c runs; `live` is false for a slot that only does its warp's work and stores nothing (the tail of
+// an unordered class, a padding slot of an ordered one: the latter repeats a unit of its key row).
+__device__ __forceinline__ int job_unit(const ExpClass& c, int g, bool& live) {
+    if (c.order) {
+        const uint32_t u = __ldg(c.order + g);
+        live = !(u & ORDER_PAD);
+        return (int)(u & ~ORDER_PAD);
+    }
+    live = g < c.count;
+    return live ? g : c.count - 1;
+}
+
+// Key-exponent loop state (keyexp classes), one register: the next window of base 0's exponent as lo * 64 + digit, lo = -1
+// once there is none.
+static_assert(KEYEXP_BITS <= 6, "the digit is packed in 6 bits");
+struct KeyWin {
+    int v;
+    __device__ __forceinline__ int lo() const { return v >> 6; }
+    __device__ __forceinline__ uint32_t entry() const { return (uint32_t)(v & 63) >> 1; }     // table entry of the odd digit
+    __device__ __forceinline__ void next(const uint32_t* e, int from) {
+        const int top = keyexp_top(e, from);
+        uint32_t d = 0;
+        v = top >= 0 ? keyexp_window(e, top, d) * 64 + (int)d : -64;
+    }
+};
+// Highest bit position of a keyexp class's merged schedule: the first window of exp[0] or the top 5-bit window of exp[1].
+__device__ __forceinline__ int keyexp_start(const KeyWin& kw, int nw1) {
+    const int p1 = (nw1 - 1) * WINDOW_BITS;
+    return kw.lo() > p1 ? kw.lo() : p1;
+}
+// Products pending at bit position p of the merged schedule: 1 = the digit of base 0 (a window ends at p), 2 = the window of
+// base 1 (p is a multiple of 5).  Worked out once per position, so that every trip of the loop runs one product.
+__device__ __forceinline__ int keyexp_pending(const KeyWin& kw, int p, int nw1) {
+    return (p == kw.lo() ? 1 : 0) | (p % WINDOW_BITS == 0 && p / WINDOW_BITS < nw1 ? 2 : 0);
+}
 
 template <int K, int TPI>
 __global__ void __launch_bounds__(128)          // (128, 4) caps at 128 registers with spills: measured 2 % slower
@@ -106,9 +147,8 @@ exp_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ tab
         int ci = 0;
         while (ci + 1 < ncls && launch->cls[ci + 1].item_begin <= (int)item) ci++;
         const ExpClass& c = launch->cls[ci];
-        const int g = ((int)item - c.item_begin) * GPW + lane / TPI;
-        const bool live = g < c.count;
-        const int i = live ? g : c.count - 1;
+        bool live;
+        const int i = job_unit(c, ((int)item - c.item_begin) * GPW + lane / TPI, live);
 
         MontCtx<L> m;
         load_operand<TPI, L>(m.n, c.mod, i);
@@ -164,10 +204,21 @@ exp_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ tab
             }
             mont_mul<TPI, L>(xr, x, m.rr, m.n, m.n0inv);
             uint32_t* tb = my_tbl + (size_t)b * TBL * K;
-            store_limbs<TPI, L>(tb, m.one);
-            store_limbs<TPI, L>(tb + K, xr);
 #pragma unroll
             for (int j = 0; j < L; j++) t[j] = xr[j];
+            if (b == 0 && c.keyexp) {
+                // odd powers: entry j = x^(2j+1), a chain with step x^2
+                mont_mul<TPI, L>(x, xr, xr, m.n, m.n0inv);
+                store_limbs<TPI, L>(tb, xr);
+#pragma unroll 1
+                for (int e = 1; e < KEYEXP_TBL; e++) {
+                    mont_mul<TPI, L>(t, t, x, m.n, m.n0inv);
+                    store_limbs<TPI, L>(tb + (size_t)e * K, t);
+                }
+                continue;
+            }
+            store_limbs<TPI, L>(tb, m.one);
+            store_limbs<TPI, L>(tb + K, xr);
 #pragma unroll 1
             for (int e = 2; e < TBL; e++) {
                 mont_mul<TPI, L>(t, t, xr, m.n, m.n0inv);
@@ -175,7 +226,36 @@ exp_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ tab
             }
         }
         __syncwarp();
-        if (c.nbases > 0) {
+        if (c.keyexp) {
+            // sliding windows over the warp's key exponent (base 0) merged with the 5-bit windows of base 1: at each bit
+            // position p a squaring, base 0's digit if a window ends at p, base 1's window if p is a multiple of 5; one product
+            // per trip (trips without a product cost as much as the saved products on the 1024-bit jobs)
+            const uint32_t* e0 = operand_at(c.exp[0], __shfl_sync(FULL, i, 0));
+            const uint32_t* e1 = c.nbases > 1 ? operand_at(c.exp[1], i) : e0;
+            const int nw1 = c.nbases > 1 ? (c.exp_limbs[1] * 32 + WINDOW_BITS - 1) / WINDOW_BITS : 0;
+            KeyWin kw;
+            kw.next(e0, c.exp_limbs[0] * 32 - 1);
+            int p = keyexp_start(kw, nw1);
+            int pend = p >= 0 ? keyexp_pending(kw, p, nw1) : 0;
+            uint32_t bb[L];
+#pragma unroll 1
+            while (pend) {                              // pend: 4 the squaring into position p, then 1 and 2 as keyexp_pending
+                if (pend & 4) {
+#pragma unroll
+                    for (int j = 0; j < L; j++) bb[j] = acc[j];
+                    pend &= 3;
+                } else if (pend & 1) {
+                    load_limbs<TPI, L>(bb, my_tbl + (size_t)kw.entry() * K);
+                    kw.next(e0, p - 1);
+                    pend &= 2;
+                } else {
+                    load_limbs<TPI, L>(bb, my_tbl + (size_t)TBL * K + (size_t)exp_window(e1, c.exp_limbs[1], p / WINDOW_BITS) * K);
+                    pend = 0;
+                }
+                mont_mul<TPI, L>(acc, acc, bb, m.n, m.n0inv);
+                if (!pend && p > 0) { p--; pend = 4 | keyexp_pending(kw, p, nw1); }
+            }
+        } else if (c.nbases > 0) {
             const uint32_t* e0 = operand_at(c.exp[0], i);
             const uint32_t* e1 = c.nbases > 1 ? operand_at(c.exp[1], i) : e0;
             const int nw0 = (c.exp_limbs[0] * 32 + WINDOW_BITS - 1) / WINDOW_BITS;
@@ -221,19 +301,25 @@ exp_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ tab
                 mont_mul<TPI, L>(acc, acc, u, m.n, m.n0inv);
             }
         }
-        if (live) store_limbs<TPI, L>(c.out + (size_t)g * c.out_stride, acc);
+        if (live) store_limbs<TPI, L>(c.out + (size_t)i * c.out_stride, acc);
         if (live && gl == 0 && work) {
             unsigned long long products = setup_products(K) + (c.nmul == 0 ? 1 : 1 + 2 * (c.nmul - 1));
             if (c.fb) {
                 for (int b = 0; b < c.nbases; b++) products += (c.exp_limbs[b] * 32 + FB_WINDOW_BITS - 1) / FB_WINDOW_BITS;
             } else if (c.nbases > 0) {
-                int nwmax = 0;
+                int nwmax = 0, first_lo = -1;
                 for (int b = 0; b < c.nbases; b++) {
                     const int nwb = (c.exp_limbs[b] * 32 + WINDOW_BITS - 1) / WINDOW_BITS;
-                    products += 1 + (TBL - 2) + nwb + ((b == 0 && c.wide0) ? 3 : 0);
+                    const int wide = (b == 0 && c.wide0) ? 3 : 0;
+                    if (b == 0 && c.keyexp) {           // x^2, 31 chain products, one product per window
+                        products += 1 + KEYEXP_TBL + keyexp_count(operand_at(c.exp[0], i), c.exp_limbs[0] * 32, first_lo) + wide;
+                        continue;
+                    }
+                    products += 1 + (TBL - 2) + nwb + wide;
                     nwmax = nwb > nwmax ? nwb : nwmax;
                 }
-                products += (unsigned long long)(nwmax - 1) * WINDOW_BITS;
+                const int top = (nwmax - 1) * WINDOW_BITS > first_lo ? (nwmax - 1) * WINDOW_BITS : first_lo;   // squarings
+                if (top > 0) products += (unsigned long long)top;
             }
             atomicAdd(work, products * mac_mont(K));
         }

@@ -250,9 +250,8 @@ nadic_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ t
         int ci = 0;
         while (ci + 1 < ncls && launch->cls[ci + 1].item_begin <= (int)item) ci++;
         const ExpClass& c = launch->cls[ci];
-        const int g = ((int)item - c.item_begin) * GPW + lane / TPI;
-        const bool live = g < c.count;
-        const int i = live ? g : c.count - 1;
+        bool live;
+        const int i = job_unit(c, ((int)item - c.item_begin) * GPW + lane / TPI, live);
 
         uint32_t n[L];
         load_operand<TPI, L>(n, c.mod, i);
@@ -272,7 +271,11 @@ nadic_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ t
             Dig<L> xr;
             to_nadic<TPI, L>(xr, is_base ? c.base[k] : c.mul[k - c.nbases], i, consts, n, n0inv);
             uint32_t* tb = my_tbl + (size_t)k * TBL * 2 * K;
-            if (is_base) {
+            const bool odd = k == 0 && c.keyexp;
+            if (odd) {
+                store_dig<TPI, L>(tb, xr);
+                Y = xr;
+            } else if (is_base) {
                 load_dig<TPI, L>(Y, consts + NADIC_ONE * K);
                 store_dig<TPI, L>(tb, Y);
                 store_dig<TPI, L>(tb + 2 * K, xr);
@@ -280,12 +283,14 @@ nadic_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ t
             } else {
                 load_dig<TPI, L>(Y, p_slot);
             }
-            // base: Y runs through xr^2 .. xr^31 into the table; multiplier: one product P *= xr
-            const int steps = is_base ? TBL - 2 : 1;
+            // base: Y runs through xr^2 .. xr^31 into the table; multiplier: one product P *= xr.  Key-exponent base 0: the
+            // first product gives x^2, which becomes the step of the chain x^3 .. x^63 of odd powers (entry j = x^(2j+1)).
+            const int steps = odd ? KEYEXP_TBL : is_base ? TBL - 2 : 1;
 #pragma unroll 1
             for (int e = 0; e < steps; e++) {
                 nadic_mul<TPI, L>(Y, Y, xr, true, n, n0inv);
-                if (is_base) store_dig<TPI, L>(tb + (size_t)(e + 2) * 2 * K, Y);
+                if (odd && e == 0) { xr = Y; load_dig<TPI, L>(Y, tb); }
+                else if (is_base) store_dig<TPI, L>(tb + (size_t)(odd ? e : e + 2) * 2 * K, Y);
             }
             if (!is_base) store_dig<TPI, L>(p_slot, Y);
         }
@@ -294,12 +299,22 @@ nadic_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ t
         // last steps of the same loop
         load_dig<TPI, L>(acc, consts + NADIC_ONE * K);
         {
-            const uint32_t* e0 = operand_at(c.exp[0], i);
+            // a keyexp class walks the sliding windows of the warp's key exponent (every lane group holds the same row)
+            const uint32_t* e0 = operand_at(c.exp[0], c.keyexp ? __shfl_sync(FULL, i, 0) : i);
             const uint32_t* e1 = c.nbases > 1 ? operand_at(c.exp[1], i) : e0;
             const int nw0 = c.nbases > 0 ? (c.exp_limbs[0] * 32 + WINDOW_BITS - 1) / WINDOW_BITS : 0;
             const int nw1 = c.nbases > 1 ? (c.exp_limbs[1] * 32 + WINDOW_BITS - 1) / WINDOW_BITS : 0;
             const int nw = nw0 > nw1 ? nw0 : nw1;
             int w = nw - 1, ph = WINDOW_BITS;
+            // keyexp: w is the bit position; ph = 8 * (next window of base 0, KeyWin) + the products pending at w (4 the squaring
+            // into w, then 1 and 2 as keyexp_pending), one per trip.  One register for both keeps the kernel at 128 registers.
+            if (c.keyexp) {
+                KeyWin kw;
+                kw.next(e0, c.exp_limbs[0] * 32 - 1);
+                w = keyexp_start(kw, nw1);
+                ph = kw.v * 8 + (w >= 0 ? keyexp_pending(kw, w, nw1) : 0);
+                if (w < 0) w = -1;
+            }
 #pragma unroll 1
             while (w >= -2) {
                 bool do_mul = true, cross2 = true;
@@ -309,6 +324,21 @@ nadic_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ t
                     for (int j = 0; j < L; j++) { Y.d0[j] = 0; Y.d1[j] = 0; }
                     if (gl == 0) Y.d0[0] = 1;
                     w = -3;
+                }
+                else if (c.keyexp) {
+                    KeyWin kw{ph >> 3};
+                    int pend = ph & 7;
+                    if (pend & 4) { square_operand<TPI, L>(Y, acc, n); cross2 = false; pend &= 3; }
+                    else if (pend & 1) { load_dig<TPI, L>(Y, my_tbl + (size_t)kw.entry() * 2 * K); kw.next(e0, w - 1); pend &= 2; }
+                    else {
+                        load_dig<TPI, L>(Y, my_tbl + ((size_t)TBL + exp_window(e1, c.exp_limbs[1], w / WINDOW_BITS)) * 2 * K);
+                        pend = 0;
+                    }
+                    if (!pend) {                        // position w done: square into w - 1, or leave for the multipliers
+                        if (w > 0) { w--; pend = 4 | keyexp_pending(kw, w, nw1); }
+                        else w = -1;
+                    }
+                    ph = kw.v * 8 + pend;
                 }
                 else if (ph < WINDOW_BITS) { square_operand<TPI, L>(Y, acc, n); cross2 = false; ph++; }
                 else if (ph == WINDOW_BITS) {
@@ -335,26 +365,29 @@ nadic_jobs_kernel(const ExpLaunch* __restrict__ launch, uint32_t* __restrict__ t
             (void)group_add_masked<TPI, L>(hi, one, 0xffffffffu);
         }
         if (live) {
-            uint32_t* o = c.out + (size_t)g * c.out_stride;
+            uint32_t* o = c.out + (size_t)i * c.out_stride;
             store_limbs<TPI, L>(o, lo);
             store_limbs<TPI, L>(o + K, hi);
             if (gl == 0 && work) {
                 // nadic_mul: 4K^2 + 2K without the second cross product (lifts, squarings), 5K^2 + 2K with it
                 const unsigned long long m4 = 4ull * K * K + 2 * K, m5 = 5ull * K * K + 2 * K;
                 unsigned long long macs = (unsigned long long)K * K + m5;                                    // exit: times (1, 0), then d0 + d1 * N
-                int nwmax = 0;
+                int nwmax = 0, first_lo = -1;
                 for (int k = 0; k < c.nbases + c.nmul; k++) {
                     const Operand& o2 = k < c.nbases ? c.base[k] : c.mul[k - c.nbases];
                     int parts = ((int)o2.limbs + K - 1) / K;
                     macs += (unsigned long long)(parts > 4 ? 4 : parts) * m4;
-                    if (k < c.nbases) {
+                    if (k == 0 && c.keyexp) {           // x^2 and 31 chain products, one product per window
+                        macs += (unsigned long long)(KEYEXP_TBL + keyexp_count(operand_at(c.exp[0], i), c.exp_limbs[0] * 32, first_lo)) * m5;
+                    } else if (k < c.nbases) {
                         const int nwb = (c.exp_limbs[k] * 32 + WINDOW_BITS - 1) / WINDOW_BITS;
                         macs += (unsigned long long)(TBL - 2 + nwb) * m5;
                         nwmax = nwb > nwmax ? nwb : nwmax;
                     } else macs += m5;
                 }
                 if (c.nmul > 0) macs += m5;
-                if (nwmax > 0) macs += (unsigned long long)(nwmax - 1) * WINDOW_BITS * m4;
+                const int top = (nwmax - 1) * WINDOW_BITS > first_lo ? (nwmax - 1) * WINDOW_BITS : first_lo;   // squarings
+                if (top > 0) macs += (unsigned long long)top * m4;
                 atomicAdd(work, macs);
             }
         }

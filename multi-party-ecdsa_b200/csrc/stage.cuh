@@ -70,7 +70,7 @@ void add_exp(ExpLaunch& l, int K, int count, Operand mod, int nb, Operand b0, Op
     ExpClass& k = l.cls[l.n_classes++];
     k.mod = mod; k.base[0] = b0; k.base[1] = b1; k.exp[0] = e0; k.exp[1] = e1; k.exp_limbs[0] = el0; k.exp_limbs[1] = el1;
     k.mul[0] = m0; k.mul[1] = m1; k.mul[2] = NONE; k.nbases = nb; k.nmul = nm; k.wide0 = 0;
-    k.fb = nullptr; k.fb_row = NONE; k.fb_sel[0] = k.fb_sel[1] = 0; k.nadic = NONE;
+    k.fb = nullptr; k.fb_row = NONE; k.fb_sel[0] = k.fb_sel[1] = 0; k.nadic = NONE; k.order = nullptr; k.keyexp = 0;
     k.out = out; k.out_stride = out_stride; k.count = count; k.item_begin = l.total_items;
     l.total_items += (count + gpw - 1) / gpw;
 }
